@@ -24,6 +24,7 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 # stdout must carry exactly one JSON line.  NCCL prints its version banner with a C-level printf to
 # fd 1 on the first communicator (seen on the 2-GPU box even with NCCL_DEBUG_FILE set), so the real
 # stdout is set aside at start-up, fd 1 is pointed at stderr for everything else this process or its
@@ -57,6 +58,7 @@ MODE_NAMES = {0: "strict_ffma", 1: "tf32", 2: "bf16x3", 3: "bf16x2", 5: "f16x2_s
 MODE_DTYPE = {0: "f32", 1: "tf32", 2: "bf16x3(split-f32)", 3: "bf16x2(split-f32)", 5: "f16x2(scaled split-f32)"}
 MODE_PRODUCTS = {2: 6, 3: 3, 5: 3}                      # tensor-core products per k-step (no roofline credit)
 MODE_TOL = {0: 1e-5, 1: 1e-3, 2: 1e-5, 3: 4e-5, 5: 1e-5}  # max |C - C_f64| / max |C_f64| (north_star bar: 1e-3)
+DUMP_ROWS = 1024              # --dump-outputs: rows of C written (16 MiB at N = 4096), shared among the ranks
 
 
 def workload_str(M, N):
@@ -126,7 +128,7 @@ def cpu_worker(kind, M, N, K, threads, steps, warmup, budget_s, timeout_s):
     for k in ("OMP_NUM_THREADS", "GOTO_NUM_THREADS", "OPENBLAS_NUM_THREADS", "MKL_NUM_THREADS"):
         env.pop(k, None)
     env["OPENBLAS_NUM_THREADS"] = str(threads)
-    cmd = [sys.executable, os.path.join(ROOT, "oracle", "cpu_ref_worker.py"), kind, str(M), str(N), str(K), str(threads),
+    cmd = [sys.executable, "-B", os.path.join(ROOT, "oracle", "cpu_ref_worker.py"), kind, str(M), str(N), str(K), str(threads),
            str(steps), str(warmup), str(budget_s)]
     try:
         r = subprocess.run(cmd, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout_s)
@@ -197,6 +199,20 @@ def cpu_baseline():
     return out
 
 
+def dump_last_step(out_dir, Cm, rank, world):
+    """C of the last timed step, as the caller receives it, for output-by-output comparison of two builds.  The
+    rows are a fixed seeded sample of the whole M = rows_per_rank * world, so they do not change between runs."""
+    import numpy as np
+    import torch
+    m = Cm.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(m * world, min(DUMP_ROWS, m * world), replace=False))
+    mine = rows[(rows >= rank * m) & (rows < (rank + 1) * m)] - rank * m
+    torch.cuda.synchronize()
+    c = Cm[torch.from_numpy(mine).to(Cm.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "c.npy" if world == 1 else f"c_rank{rank}.npy"), c)
+
+
 _T0 = time.time()
 
 
@@ -215,7 +231,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip sweep / modes / configs34 / cpu_baseline (quick runs)")
     ap.add_argument("--no-c5", action="store_true", help="skip the BASELINE configs[4] record (16384^3)")
     ap.add_argument("--slices", default="", help="K-slices of the B exchange, e.g. '512,1536,2048' (default: the plan's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help=f"write C of the last timed step as DIR/c.npy (DIR/c_rank<r>.npy with several GPUs): float32, "
+                         f"a fixed seeded sample of {DUMP_ROWS} rows of the whole C, in increasing row order")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     if args.impl == "reference":
         return run_reference(args)
@@ -329,6 +350,8 @@ def main():
     value = flops_step / (ms * 1e-3) / 1e9
     kernel_name = g.last_kernel()
     _phase("timed region done")
+    if args.dump_outputs:            # before anything below overwrites the C buffers
+        dump_last_step(args.dump_outputs, sets[(args.steps - 1) % R][2], rank, world)
 
     # ---- verification of the timed path (every rank, after the timed loop) --------------------------
     step(0)

@@ -41,7 +41,7 @@ def main():
         out_kind, what = "reference", "cuda/REF_MMult.cpp -> cblas_sgemm (vendored OpenBLAS-0.2.20, HASWELL kernels)"
     elif kind == "sgemm":
         o = _libs.load_oracle()
-        threads = o.oracle_get_threads()
+        o.oracle_set_threads(threads)
         def fn():
             c[:] = 0
             o.oracle_ref_mmult_f32_fma_fast(M, N, K, _libs.P(a), K, _libs.P(b), N, _libs.P(c), N)

@@ -2,6 +2,7 @@
 (oracle/_ref/libref.so, optional) and the product package.  Only tests/, smoke() and bench.py's
 cpu_baseline / --impl reference legs may import this."""
 import ctypes as C
+import hashlib
 import importlib
 import os
 import subprocess
@@ -17,6 +18,17 @@ PKG = "how-to-optimize-gemm_b200"
 
 def P(a):
     return a.ctypes.data_as(C.c_void_p)
+
+
+def sha256(a):
+    """SHA-256 of an array's bytes as a uint8[32]: pins a bit-exact result of any size in 32 bytes."""
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
+
+
+def seed_unseeded_drand48():
+    """Puts drand48 back in glibc's start state (X = 0), the stream a program that never seeds it draws
+    (cuda/test_MMult.cpp calls random_matrix without srand48); srand48 cannot reach that state."""
+    C.CDLL(None).seed48((C.c_ushort * 3)(0, 0, 0))
 
 
 def load_oracle():

@@ -17,14 +17,6 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    import _libs
-    if not _libs.have_ref():
-        pytest.skip("oracle/_ref/libref.so not built (needs /root/reference; run `make -C oracle ref`)")
-    return _libs.load_ref()
-
-
-@pytest.fixture(scope="session")
 def gemm():
     import _libs
     return _libs.load_pkg()
