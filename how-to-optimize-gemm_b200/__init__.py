@@ -32,6 +32,7 @@ EXPORTS = [
     "b200_gemm_debug_set_split_chunk", "b200_gemm_debug_kernel_timing", "b200_gemm_debug_kernel_time_ms",
     "b200_gemm_debug_set_cta_group", "b200_gemm_debug_set_split_tail", "b200_gemm_debug_set_group_rows",
     "b200_gemm_debug_set_ffma_variant", "b200_gemm_debug_set_epilogue", "b200_gemm_debug_set_pdl", "b200_gemm_debug_set_dynamic_sched",
+    "b200_gemm_debug_last_schedule",
 ]
 
 
@@ -105,6 +106,10 @@ lib.b200_gemm_debug_set_split_tail.argtypes = [_i]
 lib.b200_gemm_debug_set_pdl.argtypes = [_i]
 lib.b200_gemm_debug_set_dynamic_sched.argtypes = [_i]
 lib.b200_gemm_debug_kernel_time_ms.argtypes = [C.POINTER(C.c_double)]
+lib.b200_gemm_debug_last_schedule.argtypes = [C.POINTER(_i), _i]
+
+SCHEDULE_FIELDS = ("tile_m", "bn", "cta_group", "epilogue_warps", "tiles", "grid_units", "full_tiles", "split",
+                   "halfn", "dynamic")
 
 
 def kernel_time_ms():
@@ -132,6 +137,14 @@ def last_kernel():
 
 def launch_count():
     return int(lib.b200_gemm_launch_count())
+
+
+def last_schedule():
+    """Work schedule of this thread's last tensor-core or strict-FFMA launch as a dict (SCHEDULE_FIELDS), or
+    None when the last launch was another kernel (b200_gemm_debug_last_schedule)."""
+    buf = (_i * len(SCHEDULE_FIELDS))()
+    n = lib.b200_gemm_debug_last_schedule(buf, len(buf))
+    return dict(zip(SCHEDULE_FIELDS, buf[:n])) if n else None
 
 
 def _stream_ptr(stream):

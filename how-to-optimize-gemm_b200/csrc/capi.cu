@@ -48,6 +48,20 @@ struct KernelTimer {
 } g_ktimer;
 std::atomic<int> g_default_f32_mode{-1};
 thread_local const char* t_last_kernel = "none";
+// Work schedule of the calling thread's last tensor-core or FFMA launch (b200_gemm_debug_last_schedule), so that a
+// test can confirm which kernel variant and which tail path it exercised.  n = 0: the last launch was neither.
+struct SchedRecord {
+  static constexpr int N = 10;
+  int n = 0;
+  int v[N] = {};   // tile_m, bn, cta_group, epilogue_warps, tiles, grid_units, full_tiles, split, halfn, dynamic
+  void set(int tile_m, int bn, int cg, int epiw, int tiles, int units, int full, int split, int halfn, int dyn) {
+    const int r[N] = {tile_m, bn, cg, epiw, tiles, units, full, split, halfn, dyn};
+    for (int i = 0; i < N; i++) v[i] = r[i];
+    n = N;
+  }
+  void clear() { n = 0; }
+};
+thread_local SchedRecord t_last_sched;
 // General epilogue request of the current call (b200_gemm_f32_ex): read by launch_tc, reset by the entry point.
 struct EpiOpts { int axpby = 0; float alpha = 1.f, beta = 0.f; };
 thread_local EpiOpts t_epi;
@@ -270,6 +284,7 @@ int launch_zero(int m, int n, T* C, int ldc, cudaStream_t st) {
   fill_zero_kernel<T><<<grid, 256, 0, st>>>(m, n, C, ldc);
   g_launches++;
   t_last_kernel = "fill_zero";
+  t_last_sched.clear();
   return last_launch_status();
 }
 
@@ -280,6 +295,7 @@ int launch_generic(int m, int n, int k, const InT* A, int lda, const InT* B, int
   gemm_generic_kernel<InT, OutT><<<grid, 256, 0, st>>>(m, n, k, A, lda, B, ldb, C, ldc, accumulate);
   g_launches++;
   t_last_kernel = name;
+  t_last_sched.clear();
   return last_launch_status();
 }
 
@@ -289,6 +305,7 @@ int launch_generic_requant(int m, int n, int k, const int8_t* A, int lda, const 
   gemm_generic_kernel<int8_t, int8_t><<<grid, 256, 0, st>>>(m, n, k, A, lda, B, ldb, C, ldc, 0, scales, bias);
   g_launches++;
   t_last_kernel = "generic_s8_requant_64x64";
+  t_last_sched.clear();
   return last_launch_status();
 }
 
@@ -382,6 +399,7 @@ int launch_tc(int m, int n, int k, const void* A, long long lda, int a_rows_tota
   g_ktimer.end(st);
   g_launches++;
   t_last_kernel = name;
+  t_last_sched.set(Cfg::TILE_M, BN, CG, Cfg::EPI_WARPS, tiles, units, p.full_tiles, split, p.halfn, p.sched_counter != nullptr);
   return last_launch_status();
 }
 
@@ -474,7 +492,8 @@ int tc_s8_requant(int m, int n, int k, const void* A, int lda, const void* B, in
 // Workspace for the bf16 planes: cached, grow-only (no per-call cudaMalloc in steady state).  Calls
 // in split modes are serialised on this buffer by stream order; use one stream per library instance.
 // K extent accumulated inside the tensor core before folding into C (0 = whole K): [0] BF16X3, [1] BF16X2
-int g_split_chunk_k[3] = {512, 512, 1024};   // BF16X3, BF16X2, F16X2
+constexpr int kSplitChunkDefault[3] = {512, 512, 1024};   // BF16X3, BF16X2, F16X2
+int g_split_chunk_k[3] = {kSplitChunkDefault[0], kSplitChunkDefault[1], kSplitChunkDefault[2]};
 // Grows the device's split workspace to `need` bytes.  Starts at 256 MiB (every size of the reference's
 // 256..4096 sweep fits: its harness averages the first, cold call into each row, and a cudaFree +
 // cudaMalloc there costs tens of ms) and at least doubles.  Growth synchronises the device (other
@@ -736,6 +755,7 @@ int launch_ffma(int m, int n, int k, const float* A, int lda, const float* B, in
   g_ktimer.end(st);
   g_launches++;
   t_last_kernel = "ffma_128x128x32_tma";
+  t_last_sched.set(Cfg::BM, Cfg::BN, 1, 0, tiles, ctas, p.full_tiles, 1, halves, 0);
   return last_launch_status();
 }
 
@@ -766,6 +786,7 @@ int launch_ffma_fat(int m, int n, int k, const float* A, int lda, const float* B
   g_ktimer.end(st);
   g_launches++;
   t_last_kernel = "ffma_fat_128x256x32_tma";
+  t_last_sched.set(Cfg::BM, Cfg::BN, 1, 0, tiles, ctas, p.full_tiles, 1, halves, 0);
   return last_launch_status();
 }
 
@@ -864,7 +885,19 @@ void b200_gemm_debug_set_split_tail(int on) { g_split_tail = on; }
 void b200_gemm_debug_set_epilogue(int v) { g_epi_direct = v & 1; g_epi8 = ((v >> 1) & 1) ^ 1; }
 void b200_gemm_debug_set_group_rows(int rows) { g_group_rows = rows; }
 void b200_gemm_debug_set_ffma_variant(int v) { g_ffma_halves = v & 1; g_ffma_fat = v < 0 ? -1 : (v >> 1) & 1; }
-void b200_gemm_debug_set_split_chunk(int x3_k, int x2_k) { g_split_chunk_k[0] = x3_k; g_split_chunk_k[1] = x2_k; g_split_chunk_k[2] = x2_k; }
+void b200_gemm_debug_set_split_chunk(int x3_k, int x2_k) {
+  if (x3_k < 0 || x2_k < 0) {            // back to the built-in defaults, each mode its own
+    g_split_chunk_k[0] = kSplitChunkDefault[0]; g_split_chunk_k[1] = kSplitChunkDefault[1]; g_split_chunk_k[2] = kSplitChunkDefault[2];
+    return;
+  }
+  g_split_chunk_k[0] = x3_k; g_split_chunk_k[1] = x2_k; g_split_chunk_k[2] = x2_k;
+}
+int b200_gemm_debug_last_schedule(int* out, int cap) {
+  if (!out || cap <= 0) return 0;
+  const int n = t_last_sched.n < cap ? t_last_sched.n : cap;
+  for (int i = 0; i < n; i++) out[i] = t_last_sched.v[i];
+  return n;
+}
 void b200_gemm_debug_kernel_timing(int enable) { g_ktimer.on = enable != 0; g_ktimer.n = 0; }
 int b200_gemm_debug_kernel_time_ms(double* sum_ms) {
   double sum = 0;
@@ -1038,6 +1071,7 @@ int b200_gemm_f32_pack_b(int k, int n, const float* dB, int ldb, int precision_m
   b200_packed_b* h = new b200_packed_b();
   int rc = pack_operand(1, k, n, dB, ldb, precision_mode, h, (cudaStream_t)stream);
   t_last_kernel = "split_planes";
+  t_last_sched.clear();
   if (rc) { pack_release(h); delete h; return rc; }
   *out = h;
   return B200_OK;
@@ -1050,6 +1084,7 @@ int b200_gemm_f32_pack_a(int m, int k, const float* dA, int lda, int precision_m
   b200_packed_a* h = new b200_packed_a();
   int rc = pack_operand(0, m, k, dA, lda, precision_mode, h, (cudaStream_t)stream);
   t_last_kernel = "split_planes";
+  t_last_sched.clear();
   if (rc) { pack_release(h); delete h; return rc; }
   *out = h;
   return B200_OK;
@@ -1133,6 +1168,7 @@ int b200_mxf4_quantize_a(int m, int k, const float* dA, int lda, uint8_t* dQ, ui
   mxf4_quantize_rows_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(dA, lda, m, k, dQ, kpad, dSF, rows_pad);
   g_launches++;
   t_last_kernel = "mxf4_quantize_rows";
+  t_last_sched.clear();
   return last_launch_status();
 }
 
@@ -1146,6 +1182,7 @@ int b200_mxf4_quantize_b(int k, int n, const float* dB, int ldb, uint8_t* dQ, ui
   mxf4_quantize_cols_t_kernel<<<dim3((n_pad + 255) / 256, kpad / 32), 256, 0, (cudaStream_t)stream>>>(dB, ldb, k, n, dQ, kpad, dSF, n_pad);
   g_launches++;
   t_last_kernel = "mxf4_quantize_cols_t";
+  t_last_sched.clear();
   return last_launch_status();
 }
 
@@ -1179,6 +1216,7 @@ int b200_gemm_mxf4(int m, int n, int k, const uint8_t* dAq, const uint8_t* dSFA,
   g_ktimer.end(st);
   g_launches++;
   t_last_kernel = "tc_mxf4_128x128";
+  t_last_sched.clear();
   return last_launch_status();
 }
 
@@ -1192,6 +1230,7 @@ int b200_convert_f32_to_bf16(const float* dSrc, uint16_t* dDst, size_t count, vo
   convert_f32_to_bf16_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(dSrc, dDst, count);
   g_launches++;
   t_last_kernel = "convert_f32_to_bf16";
+  t_last_sched.clear();
   return last_launch_status();
 }
 

@@ -278,8 +278,9 @@ void b200_gemm_debug_set_b_desc(int lbo_bytes, int sbo_bytes);
  * pre-pass kernels are launched with the programmatic-serialisation attribute and order themselves with
  * griddepcontrol.wait, so a kernel's prologue overlaps the tail of its predecessor in the stream). */
 void b200_gemm_debug_set_pdl(int mask);   /* bit 0: PDL on; bit 1: keep the F16X2 pre-pass of B on the caller's stream (default: auxiliary stream beside A's) */
-/* Tuning hook: 0 = static round-robin tile schedule (default 1: a scheduler warp hands tiles out from an atomic
- * counter, so CTAs that start late because a co-running kernel holds their SM draw fewer tiles). */
+/* Tuning hook: 1 = a scheduler warp hands tiles out from an atomic counter, so CTAs that start late because a
+ * co-running kernel holds their SM draw fewer tiles; 0 (default) = static round-robin tile schedule, except where
+ * the row-panel plan asks for the dynamic one. */
 void b200_gemm_debug_set_dynamic_sched(int on);
 /* Tuning hook: force the tensor-core tile width (128, 192 or 256; 0 = built-in heuristic). */
 void b200_gemm_debug_set_bn(int bn);
@@ -289,8 +290,18 @@ void b200_gemm_debug_set_cta_group(int cg);
  * CTAs and folded into C in order; 0 = whole tiles only. */
 void b200_gemm_debug_set_split_tail(int on);
 /* Tuning hook: K extent the tensor core accumulates before the epilogue folds the partial sum
- * into C with a rounded fp32 add (two-level accumulation of the split modes); 0 = whole K. */
+ * into C with a rounded fp32 add (two-level accumulation of the split modes); 0 = whole K.
+ * bf16x2_k sets the F16X2 mode's extent as well.  A negative argument restores the built-in
+ * defaults of all three modes (BF16X3 512, BF16X2 512, F16X2 1024). */
 void b200_gemm_debug_set_split_chunk(int bf16x3_k, int bf16x2_k);
+/* Test hook: the work schedule of the calling thread's last tensor-core or strict-FFMA kernel launch, as
+ * {tile_m, bn, cta_group, epilogue_warps, tiles, grid_units, full_tiles, split, halfn, dynamic}:
+ * rows and columns of one tile (tile_m = 256 for a CTA pair), CTAs per tile, epilogue warps per CTA
+ * (0 for the FFMA kernels), tiles of C, CTAs or CTA pairs launched, work items that are whole tiles,
+ * K parts of each tail tile, 1 if tail tiles are issued as two half-width tiles (the FFMA kernels'
+ * half tiles), 1 if the dynamic tile scheduler ran.  Writes min(10, cap) values to out and returns the
+ * count; returns 0 when the last launch of the thread was another kernel (generic, fill, pre-pass). */
+int  b200_gemm_debug_last_schedule(int* out, int cap);
 /* Tuning hook: rows of A per raster group of the persistent tile schedule (0 = 2048). */
 void b200_gemm_debug_set_group_rows(int rows);
 /* Tuning hook for the strict fp32 kernels: bit 0 = half tiles in the last partial round (default on),
